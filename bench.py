@@ -701,24 +701,31 @@ def run_single(args, rank, world, local_rank, dist, cpu_arm=True):
     blind_wall_us = {q: [] for q in QUERIES}
     e2e_us = {q: [] for q in QUERIES}
     resident = {}
+    blind_rows = {}
     eng.set_profiling(1)
     for _ in range(args.steps):
         for q in QUERIES:
             pats, nvars, req = plans[q]
-            w, d, _, _ = host.time_query(eng, pats, nvars, req, 1, blind=True, flush=True, device_times=True)
+            w, d, blind_rows[q], _ = host.time_query(eng, pats, nvars, req, 1, blind=True, flush=True, device_times=True)
             dev_us[q].append(float(d[0]))
             blind_wall_us[q].append(float(w[0]))
             resident[q] = bool(eng.get_option(capi.WK_INFO_LAST_RESIDENT))
     eng.set_profiling(0)
-    for _ in range(args.steps):
+    dump = args.dump_outputs if rank == 0 else ""
+    tables = {}
+    for step in range(args.steps):
         for q in QUERIES:
             pats, nvars, req = plans[q]
-            w, _, _, _ = host.time_query(eng, pats, nvars, req, 1, blind=False, table=out_tbl, flush=True)
+            w, _, r, c = host.time_query(eng, pats, nvars, req, 1, blind=False, table=out_tbl, flush=True)
             e2e_us[q].append(float(w[0]))
+            if dump and step == args.steps - 1:     # the next query overwrites out_tbl; its clock starts after this copy
+                tables[q] = out_tbl[: r * c].reshape(r, c).copy()
     barrier()
     t_region = time.time() - t_region0
     clocks = sampler.stop()
     launches = eng.launch_count() - launches0
+    if dump:
+        dump_outputs(dump, tables, blind_rows)
 
     # ---- the tables themselves (not only their sizes): digest of every query's non-blind result -----------------
     digests = {}
@@ -832,6 +839,30 @@ def run_single(args, rank, world, local_rank, dist, cpu_arm=True):
     return line if rank == 0 else None
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(d, tables, rows):
+    """--dump-outputs: what the end-to-end path handed back in the last timed step, so that two builds can be compared output
+    for output.  DIR/q<N>.npy is query N's result table as float64 (exact for every 32-bit id) with its rows in lexicographic
+    order (the engine returns them in no fixed order); a query without an answer has no file.  DIR/rows.npy holds the row
+    counts of Q1..Q7.  Should the tables exceed 64 MB in all, each keeps the same fraction of its sorted rows (at least one),
+    drawn with a fixed seed."""
+    import sparql_mini as M
+    os.makedirs(d, exist_ok=True)
+    total = 8 * sum(t.size for t in tables.values())
+    frac = min(1.0, (DUMP_BYTES - 4096 * (len(tables) + 1)) / total) if total else 1.0
+    for q, t in sorted(tables.items()):
+        if t.size == 0:
+            continue
+        t = M.sort_rows(t)
+        if frac < 1.0:
+            keep = max(1, int(t.shape[0] * frac))
+            t = t[np.sort(np.random.default_rng(q).choice(t.shape[0], keep, replace=False))]
+        np.save(os.path.join(d, "q%d.npy" % q), t.astype(np.float64))
+    np.save(os.path.join(d, "rows.npy"), np.array([rows[q] for q in QUERIES], dtype=np.float64))
+
+
 def ncu_traffic(args, q, step, kind):
     """DRAM traffic per launch (dram__bytes_read.sum + dram__bytes_write.sum) of this launch from the committed ncu --set full
     capture of the same command (profiles/ncu_traffic.json, see profiles/README.md); None when no capture of this workload /
@@ -888,7 +919,12 @@ def main():
     ap.add_argument("--mode", default="auto", choices=["auto", "replicas", "sharded"],
                     help="N>1: sharded (vid %% N, exchange over NVLink; the default) or replicas (whole store per GPU, weak scaling)")
     ap.add_argument("--no-secondary", action="store_true", help="N>1 sharded: skip the single-GPU run of the same store and the replicas run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the result tables of the last end-to-end step as DIR/q<N>.npy (float64, rows "
+                         "sorted; no file for a query without an answer) and the row counts as DIR/rows.npy; one GPU or replicas only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -896,6 +932,8 @@ def main():
     if args.mode == "auto":
         args.mode = "sharded" if args.gpus > 1 else "replicas"
     sharded = args.gpus > 1 and args.mode == "sharded"
+    if args.dump_outputs and (sharded or args.impl == "reference"):
+        ap.error("--dump-outputs writes the GPU path's tables of one GPU or of replicas, not of the sharded mode or the reference arm")
     if not args.scale:
         args.scale = 10240 if sharded else 2560     # BASELINE configs 4 and 3
     if not args.plan:

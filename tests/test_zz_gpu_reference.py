@@ -1,10 +1,12 @@
-"""GPU: the engine against the reference's OWN compiled code (green on the B200 since the driver's round-1 run and in every
-1-GPU call of round 2; the file name sorts last for historical reasons).
+"""GPU: the engine against the answers of the reference's OWN compiled code (the file name sorts last for historical
+reasons), all of them committed under tests/golden/ (made from oracle/_ref by make_ref_engine.py and make_ref_checks.py):
 
-* the committed answers of the reference engine (tests/golden/ref_engine_lubm1.json, made by tests/golden/make_ref_engine.py
-  from oracle/_ref) -- always runs;
+* the reference engine's answers on LUBM-1 and LUBM-2 (ref_engine_lubm{1,2}.json);
 * a store BUILT BY THE REFERENCE (StaticGStore::init, CPU build with many 256-bucket ext extents, unsorted index lists),
-  uploaded as is with wk_store_create and queried on the GPU -- runs when oracle/_ref travelled with the snapshot."""
+  uploaded as is with wk_store_create and queried on the GPU (ref_store_lubm1_head.npz);
+* the reference engine's answers on a random graph (ref_checks.json)."""
+import os
+
 import numpy as np
 import pytest
 
@@ -14,6 +16,7 @@ from oracle import oracle as O
 from wukong_b200 import capi
 
 pytestmark = pytest.mark.gpu
+HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 @pytest.fixture(scope="module")
@@ -52,53 +55,60 @@ def test_matches_reference_engine_fixture(eng1, eng2, which):
             assert hashlib.sha256(np.ascontiguousarray(tbl).tobytes()).hexdigest() == e["distinct_sha256"], name
 
 
-def test_reference_built_store_runs_on_the_gpu(lubm1, ostore1):
-    from oracle import ref as REF
-    try:
-        ok = REF.available()
-    except OSError:
-        ok = False
-    if not ok:
-        pytest.skip("oracle/_ref not present on this box")
-    rs = REF.RefStore(lubm1)
+LUBM_HEAD = 10000     # the first triples of LUBM-1: a reference-built store of all of it does not fit a small test vector
+
+
+def reference_built_store():
+    """the store arrays the reference's StaticGStore::init builds for lubm1[:LUBM_HEAD] (tests/golden/ref_store_lubm1_head.npz,
+    made by tests/golden/make_ref_checks.py from oracle/_ref; only the occupied header slots are stored)"""
+    z = np.load(os.path.join(HERE, "golden", "ref_store_lubm1_head.npz"))
+    v = np.zeros((int(z["num_slots"][0]), 2), dtype=np.uint64)
+    v[z["slots"], 0], v[z["slots"], 1] = z["keys"], z["ptrs"]
+    return v, z["edges"], z["segs"]
+
+
+def test_reference_built_store_runs_on_the_gpu(lubm1):
+    """a store BUILT BY THE REFERENCE (CPU build with many 256-bucket ext extents, unsorted index lists) uploaded as is with
+    wk_store_create and queried on the GPU: Q1-Q7 x 3 plan sets against the oracle on the same triples"""
+    tr = lubm1[:LUBM_HEAD]
+    ost = O.Store.build(tr, kvstore_bytes=32 << 20, num_engines=4)
+    v, e, rsegs = reference_built_store()
     segs = []
-    for r in rs.segs():
+    for r in rsegs:
         m = capi.SegMeta()
         m.index, m.dir, m.pid = int(r[0]), int(r[1]), int(r[2])
         m.num_keys, m.num_buckets, m.bucket_start, m.num_edges, m.edge_start = (int(x) for x in r[3:8])
         m.ext_start, m.ext_num = int(r[9]), int(r[10])        # first extent only (informational: probes follow chain pointers)
         segs.append(m)
-    v = rs.vertices()
     v = v[: (v.shape[0] // 8) * 8]      # GStore's slot count need not be a multiple of 8; no bucket id reaches the partial tail
-    gst = capi.Store(v, rs.edges(), segs)
+    gst = capi.Store(v, e, segs)
     eng = capi.Engine(gst, rbuf_bytes=64 << 20)
+    nonempty = 0
     for q in range(1, 8):
         for plan in PLANS:
             pats, nvars, req, _ = load_query(q, plan)
-            want = O.run_query([ostore1], pats, nvars, req)
+            want = O.run_query([ost], pats, nvars, req)
             rc, rows, cols, tbl = eng.query(pats, nvars, req)
             assert rc == 0 and rows == want.rows, (q, plan)
             if rows:
+                nonempty += 1
                 assert rows_equal(tbl, want.table), (q, plan)
-    s, p, o = (int(x) for x in lubm1[4321])
-    assert np.array_equal(gst.get_edges(s, p, O.OUT), rs.get_edges(s, p, O.OUT))
+    assert nonempty == 18          # Q3 has no answer on these triples
+    s, p, o = (int(x) for x in tr[4321])
+    assert np.array_equal(gst.get_edges(s, p, O.OUT), ost.get_edges(s, p, O.OUT))
     eng.close()
     gst.close()
 
 
 def test_random_graph_against_live_reference_engine():
-    """a random graph (tests/random_bgp.py) answered by the GPU engine and, live, by the reference's compiled engine"""
+    """a random graph (tests/random_bgp.py) answered by the GPU engine and by the reference's compiled engine (its answers are
+    committed in tests/golden/ref_checks.json, made by tests/golden/make_ref_checks.py)"""
+    import hashlib
+    import json
     import random_bgp as R
-    from oracle import ref as REF
-    try:
-        ok = REF.available()
-    except OSError:
-        ok = False
-    if not ok:
-        pytest.skip("oracle/_ref not present on this box")
+    gold = json.load(open(os.path.join(HERE, "golden", "ref_checks.json")))["gpu_random_graph"]
     tr, meta = R.graph(0, nv=400, ntriples=4000)
     npreds = meta["num_normal_preds"]
-    rs = REF.RefStore(tr, num_normal_preds=npreds)
     gst = capi.Store.build(tr, npreds)
     eng = capi.Engine(gst, rbuf_bytes=256 << 20)
     checked = 0
@@ -107,8 +117,9 @@ def test_random_graph_against_live_reference_engine():
         rc, rows, cols, tbl = eng.query(planned, nvars, req)
         if rc == capi.WK_ERR_RBUF_OVERFLOW or rows > 300_000:
             continue
-        rrc, rrows, _, rtbl = rs.query(planned, nvars, req)
-        assert rc == 0 and rrc == 0 and rrows == rows and (rows == 0 or rows_equal(tbl, rtbl)), (qseed, planned)
+        g = gold["q%d" % qseed]
+        assert rc == 0 and g["rc"] == 0 and g["rows"] == rows, (qseed, planned)
+        assert rows == 0 or hashlib.sha256(M.sort_rows(tbl).tobytes()).hexdigest() == g["sha256"], (qseed, planned)
         checked += 1
     assert checked >= 30
     eng.close()
